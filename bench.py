@@ -355,6 +355,18 @@ def run_cfg3(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, blocks):
+    """Writes the label blocks one step of the timed path returned (`TorchSeqRecognizer.collect`: counts, labels, starts, ends,
+    confs) as DIR/<name>.npy, integers as float64 and confidences as float32.  The engine leaves the slots past a line's count
+    unwritten, so they are zeroed: two runs on the same inputs then compare element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    valid = np.arange(blocks['labels'].shape[1])[None, :] < blocks['counts'][:, None]
+    for name, a in blocks.items():
+        if a.ndim == 2:
+            a = np.where(valid, a, 0)
+        np.save(os.path.join(out_dir, name + '.npy'), a.astype(np.float32 if name == 'confs' else np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -369,7 +381,13 @@ def main():
     ap.add_argument('--workload', default='cfg2', choices=['cfg2', 'cfg3'])
     ap.add_argument('--pages', type=int, default=8)
     ap.add_argument('--cfg5-lines', type=int, default=100000)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the label blocks of the last timed `value` step (rank 0) to DIR/<name>.npy (cfg2 GPU arm only)')
     args = ap.parse_args()
+    if args.dump_outputs is not None and (args.impl != 'b200' or args.workload != 'cfg2'):
+        ap.error('--dump-outputs applies to the cfg2 workload of the GPU arm')
+    if args.steps is not None and args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     if args.steps is None:
         args.steps = 200 if (args.impl == 'b200' and args.workload == 'cfg2') else 20
@@ -510,6 +528,8 @@ def main():
     m.reset_launch_count()
     ms_total, rb_value = timed(devb, args.steps, pipelined=True)
     launches = m.launch_count
+    # the e2e regions below write into the same result buffer: keep what the last `value` step returned
+    last_value = {k: v.copy() for k, v in rb_value.views(args.steps - 1).items()}
     # ---- timed region 3: end to end through the public API with pinned host buffers
     ms_e2e_serial, _ = timed(host, args.steps)
     ms_e2e, _ = timed(host, args.steps, pipelined=True)
@@ -550,6 +570,9 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, last_value)
 
     pk = peaks()
     work = stage_work()

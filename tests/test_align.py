@@ -1,8 +1,9 @@
 """Forced alignment (SURVEY 8f rank 4: the `return_logits` consumer, kraken/tasks/align.py:111-137).
 
-CPU: oracle/align_oracle.py against the reference's own get_trellis / backtrack / merge_repeats (bit for bit; skipped where
-/root/reference is absent) and against the committed goldens generated from the reference (tests/golden/align_cases.npz).
+CPU: oracle/align_oracle.py against the outputs of the reference's own get_trellis / backtrack / merge_repeats (bit for bit,
+tests/golden/ref_align.npz) and against the committed goldens generated from the reference (tests/golden/align_cases.npz).
 GPU: `kb_forced_align` through the C ABI against the oracle - token indices and frame ranges exact, scores within 1e-5."""
+import hashlib
 import os
 
 import numpy as np
@@ -27,41 +28,45 @@ def random_case(rng, C, T, J, peaky=True):
     return p, [int(t) for t in tokens]
 
 
-def reference_align(p, tokens):
-    from kraken.tasks import align as ra
-    labels = torch.tensor(tokens, dtype=torch.int32).long()
-    em = p.squeeze().log_softmax(0).T
-    tr = ra.get_trellis(em, labels)
-    try:
-        path = ra.backtrack(tr, em, labels)
-    except ValueError:
-        return tr, None, None
-    segs = ra.merge_repeats(path, list(range(len(tokens))))          # "ground truth" = the token indices: Segment.label = index
-    return tr, path, segs
-
-
 def test_oracle_is_the_reference_bit_for_bit():
-    import refshim
-    if not refshim.available():
-        pytest.skip('reference tree not present')
-    refshim.install()
+    """120 random cases against the reference's get_trellis / backtrack / merge_repeats on them (tests/golden/ref_align.npz, generated
+    by oracle/make_reference_checks.py).  Where this CPU's torch softmax reproduces the reference's probabilities bit for bit, the
+    trellis (sha256 of its bytes), path and segments are compared exactly.  Elsewhere the probabilities and emissions differ in the
+    last bits: token and frame indices stay exact, the trellis sum and the scores agree to float32 rounding."""
+    g = np.load(os.path.join(os.path.dirname(GOLDEN), 'ref_align.npz'))
     rng = np.random.default_rng(0)
-    n_failed = 0
-    for it in range(120):
+    n_failed, n_exact, pi, si = 0, 0, 0, 0
+    for it in range(len(g['path_n'])):
         C = int(rng.integers(3, 60)); T = int(rng.integers(4, 160)); J = int(rng.integers(1, max(2, T // 2)))
         p, tokens = random_case(rng, C, T, J, peaky=bool(it % 3))
-        rtr, rpath, rsegs = reference_align(p, tokens)
+        exact = hashlib.sha256(p.numpy().tobytes()).digest() == g['probs_sha'][it].tobytes()
+        n_exact += exact
         em = ao.emission_from_probs(p)
         tr = ao.trellis(em, tokens)
-        assert torch.equal(torch.from_numpy(tr), rtr), it
+        assert tr.shape == tuple(g['trellis_shape'][it]), it
+        if exact:
+            assert hashlib.sha256(tr.tobytes()).digest() == g['trellis_sha'][it].tobytes(), it
+        assert np.isclose(tr[np.isfinite(tr)].astype(np.float64).sum(), g['trellis_sum'][it], rtol=1e-6, atol=1e-4), it
         path = ao.backtrack(tr, em, tokens)
-        if rpath is None:
+        npath, nsegs = int(g['path_n'][it]), int(g['segs_n'][it])
+        if npath < 0:
             assert path is None
             n_failed += 1
             continue
-        assert path == [(q.token_index, q.time_index, q.score) for q in rpath], it
-        assert ao.merge_repeats(path) == [(s.label, s.start, s.end, s.score) for s in rsegs], it
-    assert n_failed < 120
+        want = [(int(a), int(b), float(s)) for (a, b), s in zip(g['path_ij'][pi:pi + npath], g['path_score'][pi:pi + npath])]
+        segs = ao.merge_repeats(path)
+        want_segs = [(int(a), int(b), int(c), float(s)) for (a, b, c), s in zip(g['seg_lse'][si:si + nsegs], g['seg_score'][si:si + nsegs])]
+        if exact:
+            assert path == want, it
+            assert segs == want_segs, it
+        else:
+            assert [q[:2] for q in path] == [q[:2] for q in want], it
+            assert np.allclose([q[2] for q in path], [q[2] for q in want], rtol=1e-6, atol=0), it
+            assert [s[:3] for s in segs] == [s[:3] for s in want_segs], it
+            assert np.allclose([s[3] for s in segs], [s[3] for s in want_segs], rtol=1e-6, atol=0), it
+        pi, si = pi + npath, si + nsegs
+    assert it == 119 and n_failed < 120 and pi == len(g['path_ij']) and si == len(g['seg_lse'])
+    print(f'{n_exact} of 120 cases with bit-identical probabilities')
 
 
 def test_oracle_against_the_goldens():

@@ -41,3 +41,28 @@ def test_per_stage_roofline_arithmetic():
     fl = 2 * 200 * 768 * 2048 * 64
     assert abs(r['L_5.xproj']['tflops'] - fl / 1e-4 / 1e12) < 0.01 and abs(r['L_5.xproj']['tensor_frac'] - r['L_5.xproj']['tflops'] / 1000.0) < 1e-3
     assert r['decode']['tflops'] == 0 and r['decode']['gbs'] > 0
+
+
+def test_dump_outputs_writes_float_arrays_with_unwritten_slots_zeroed(tmp_path):
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import bench
+    from kraken_b200.dist import ResultBlocks
+    rb = ResultBlocks(2, 3, 5, pin=False)
+    rb.t.fill_(7)                                            # stands for whatever an earlier run left in the buffer
+    v = rb.views(1)
+    v['counts'][:] = [0, 2, 5]
+    v['labels'][1, :2] = [4, 9]; v['starts'][1, :2] = [0, 3]; v['ends'][1, :2] = [1, 4]; v['confs'][1, :2] = [0.5, 0.25]
+    bench.dump_outputs(str(tmp_path / 'out'), {k: a.copy() for k, a in v.items()})
+    got = {f[:-4]: np.load(tmp_path / 'out' / f) for f in os.listdir(tmp_path / 'out')}
+    assert sorted(got) == ['confs', 'counts', 'ends', 'labels', 'starts']
+    assert got['confs'].dtype == np.float32 and all(got[k].dtype == np.float64 for k in ('counts', 'labels', 'starts', 'ends'))
+    assert got['counts'].tolist() == [0, 2, 5]
+    assert got['labels'][0].tolist() == [0] * 5 and got['labels'][1].tolist() == [4, 9, 0, 0, 0] and got['labels'][2].tolist() == [7] * 5
+    assert got['confs'][1].tolist() == [0.5, 0.25, 0, 0, 0]
+
+
+def test_dump_outputs_only_for_the_gpu_cfg2_arm():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--impl', 'reference', '--dump-outputs', 'unused'],
+                       capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert p.returncode == 2 and '--dump-outputs' in p.stderr and not os.path.exists(os.path.join(ROOT, 'unused'))

@@ -1,6 +1,5 @@
 """Native readers of kraken's on-disk formats (kraken_b200/weights.py; replaces kraken/models/loaders.py:46-254 and
-kraken/models/_coreml.py for the engine).  Synthetic files always; the reference's own fixtures when the checkout is mounted
-(build container only)."""
+kraken/models/_coreml.py for the engine): synthetic files, and the reference's own model files (copies in tests/golden)."""
 import json
 import os
 import struct
@@ -10,8 +9,7 @@ import pytest
 
 from kraken_b200.weights import load_coreml, load_model_file, load_safetensors
 
-RES = '/root/reference/tests/resources'
-needs_ref = pytest.mark.skipif(not os.path.isdir(RES), reason='reference checkout not mounted')
+RES = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 
 
 def write_safetensors(path, tensors, metadata):
@@ -71,7 +69,6 @@ def test_safetensors_error_paths(tmp_path):
         load_safetensors(p)                                              # no VGSL spec
 
 
-@needs_ref
 def test_reference_fixtures_fp16_and_coreml():
     a = load_safetensors(os.path.join(RES, 'model_small.safetensors'))[0]
     c = load_safetensors(os.path.join(RES, 'model_small_fp16.safetensors'))[0]
@@ -87,7 +84,6 @@ def test_reference_fixtures_fp16_and_coreml():
         load_coreml(os.path.join(RES, 'model_small.mlmodel'))             # (kraken/models/loaders.py:195-200)
 
 
-@needs_ref
 def test_model_object_from_file_matches_reference_surface():
     import kraken_b200 as kb
     m = kb.TorchVGSLModel.load_model(os.path.join(RES, 'overfit.mlmodel'))
